@@ -39,6 +39,7 @@ FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 WORKLOAD = "base_sca"
 WORKLOAD_TEXT = ("base_sca: MultiScaleDeformableAttn 200x200 BEV (40000 queries), 6 cams, 4 levels "
                  "[[116,200],[58,100],[29,50],[15,25]], 8 heads x 32 ch, 4x8 points (BASELINE configs[2])")
+DUMP_QUERIES = 4096  # 6 cameras x 4096 queries x 8 heads x 32 channels in float32: 25 MB
 DIST_TEXT = {"U": "U: reference unit-test distribution (all points in range, worst case)",
              "G": "G: camera-ring geometry (~1/6 of camera x query pairs visible)"}
 
@@ -97,7 +98,13 @@ def parse():
                          "step's tensors during warm-up")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary (other distribution / INT8) legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="1 GPU: after the timed steps, write the output of the last one to DIR/msda_output.npy (float32; "
+                         f"a fixed, seeded sample of {DUMP_QUERIES} BEV queries, every camera, head and channel)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def ncu_traffic(key):
@@ -344,6 +351,17 @@ def time_kernel(fn, steps, warmup, flush=None):
     return sum(per), per
 
 
+def dump_outputs(out_dir, y):
+    """Writes the plugin op's output y [cameras, queries, heads, channels] (what a caller of the timed path receives) for
+    comparing two builds output for output. The whole tensor is 245 MB in float32, so the same seeded sample of
+    queries is taken every run."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    q = torch.randperm(y.shape[1], generator=torch.Generator().manual_seed(0))[:DUMP_QUERIES].sort().values
+    np.save(os.path.join(out_dir, "msda_output.npy"), y[:, q.to(y.device)].float().cpu().numpy())
+
+
 def run_single(args, cfg, peak, peak_src):
     from bevformer_tensorrt_b200 import _lib
     from bevformer_tensorrt_b200.workloads import make_msda_inputs
@@ -372,7 +390,10 @@ def run_single(args, cfg, peak, peak_src):
         for _ in range(args.steps):
             if flush is not None:
                 flush.zero_()
-            fn()
+            if args.dump_outputs:
+                last = fn()
+            else:
+                fn()
         end.record()
         torch.cuda.synchronize()
         total_ms = start.elapsed_time(end)
@@ -382,6 +403,9 @@ def run_single(args, cfg, peak, peak_src):
         while time.perf_counter() - t_wall0 < 1.0:
             fn()
         torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+        del last
     ms_step = total_ms / args.steps
     # per-launch duration of the dominant (only) kernel, measured live with events around each launch
     _, per = time_kernel(fn, min(args.steps, 50), 3, flush)
@@ -833,6 +857,8 @@ def main():
         raise SystemExit("bench.py: no CUDA device. The product path has no CPU fallback; run under gpurun.")
     peak, peak_src = hbm_peak()
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world > 1 and args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs writes the 1-GPU step's output; run it with --gpus 1")
     if world > 1:
         # NCCL prints its version banner to stdout at communicator creation when the box sets NCCL_DEBUG=VERSION; the
         # contract is ONE JSON line on stdout, so everything the run itself emits goes to stderr until the line is ready

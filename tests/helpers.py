@@ -18,6 +18,21 @@ def input_digest(*tensors):
     return h.hexdigest()
 
 
+def sample_index(numel, k, seed=0):
+    """Sorted flat indices of a fixed, seeded sample of about k elements of an output with numel elements (the form in
+    which tests/golden stores outputs too large for a fixture)."""
+    return np.unique(np.random.default_rng(seed).integers(0, numel, k))
+
+
+def load_ref_kernels(name):
+    """Outputs of the reference's own CUDA kernels (tests/golden/make_golden_ref_kernels.py)."""
+    return np.load(os.path.join(GOLDEN, f"ref_kernels_{name}.npz"))
+
+
+def check_digest(z, key, *tensors):
+    assert input_digest(*tensors) == str(z[f"{key}_digest"]), f"{key}: the seeded inputs no longer match the fixture"
+
+
 def golden_msda_cases():
     return sorted(glob.glob(os.path.join(GOLDEN, "msda_*.npz")))
 

@@ -1,5 +1,5 @@
 """GPU parity tests for the grid sampler (pytest -m gpu). Checkers: oracle/grid_sampler_oracle.c (the reference FP32
-kernel restated), golden vectors from the reference Python binding, and oracle/_ref (the reference's CUDA kernels).
+kernel restated), golden vectors from the reference Python binding and from the reference's CUDA kernels run on a B200.
 Tolerances: FP32 1e-5; FP16 1e-3 + output rounding slack for |out| > 2 (bicubic overshoots); INT8 2e-2-style bound in
 units of the output scale."""
 import itertools
@@ -12,9 +12,9 @@ import torch
 import bevformer_tensorrt_b200 as bt
 from bevformer_tensorrt_b200.functions.grid_sampler import pack_chw, unpack_chw
 from bevformer_tensorrt_b200.workloads import quantize_per_tensor
-from oracle import REF_LIB
 from oracle import grid_sampler as ogs
-from tests.helpers import GOLDEN, make_grid_sampler_inputs, make_rotation_grid
+from tests.helpers import (GOLDEN, check_digest, load_ref_kernels, make_grid_sampler_inputs, make_rotation_grid,
+                           sample_index)
 
 pytestmark = pytest.mark.gpu
 
@@ -186,42 +186,25 @@ def test_base_shape_identity_and_shift_properties():
     assert np.abs(outh.float().cpu().numpy() - want).max() < 1e-3 + np.abs(want).max() * 2.0**-11
 
 
-needs_ref = pytest.mark.skipif(not os.path.exists(REF_LIB), reason="oracle/_ref not built")
+# the reference's own CUDA kernels, run on a B200 (tests/golden/ref_kernels_grid_sampler.npz, make_golden_ref_kernels.py)
+REFK = load_ref_kernels("grid_sampler")
 
 
-@needs_ref
 @pytest.mark.parametrize("interp,pad,align", MODES)
 def test_fp32_matches_reference_kernel(interp, pad, align):
-    import ctypes
-
+    """Against the reference's grid_sample<float> on a fixed, seeded sample of the output elements."""
     inp, grid = make_grid_sampler_inputs(2, 5, 17, 19, 33, 31, seed=9)
-    inp, grid = inp.cuda(), grid.cuda()
-    lib = ctypes.CDLL(REF_LIB)
-    out = torch.empty(2, 5, 33, 31, device="cuda")
-    dims = lambda t: (ctypes.c_int * 4)(*t.shape)  # noqa: E731
-    lib.ref_grid_sample(0, ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(inp.data_ptr()),
-                        ctypes.c_void_p(grid.data_ptr()), dims(out), dims(inp), dims(grid), 4, IM[interp], PM[pad],
-                        int(align), ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))  # fmt: skip
-    torch.cuda.synchronize()
-    got = bt.grid_sampler(inp, grid, interp, pad, align)
-    assert (got - out).abs().max().item() < 1e-5, (interp, pad, align)
-
-
-def _ref_call(name, *args):
-    import ctypes
-
-    lib = ctypes.CDLL(REF_LIB)
-    getattr(lib, name)(*args, ctypes.c_void_p(torch.cuda.current_stream().cuda_stream))
-    torch.cuda.synchronize()
+    check_digest(REFK, "fp32", inp, grid)
+    got = bt.grid_sampler(inp.cuda(), grid.cuda(), interp, pad, align).cpu().numpy().reshape(-1)
+    want = REFK[f"fp32_{interp}_{pad}_{int(align)}"]
+    assert np.abs(got[sample_index(got.size, 512)] - want).max() < 1e-5, (interp, pad, align)
 
 
 def test_base_shape_fp16_config4_vs_oracle_and_reference_kernel():
     """BASELINE configs[3], FP16 leg: prev-BEV warp [1,256,200,200] through a rotation grid, bilinear / zeros /
     align_corners=False, every output element vs the CPU oracle (reference FP32 formulas, gridSamplerKernel.cu:666-795,
-    on the fp16-rounded tensors); kLINEAR and kCHW2 entries; the reference's own __half / __half2 kernels
-    (:797-1080, coordinates in half precision) are run beside it on the same tensors and reported."""
-    import ctypes
-
+    on the fp16-rounded tensors); kLINEAR and kCHW2 entries; the reference's own __half kernel (:797-1080, coordinates
+    in half precision) on the same tensors, run on a B200 (REFK), must not come closer to those formulas."""
     g = torch.Generator().manual_seed(21)
     x = torch.randn(1, 256, 200, 200, generator=g).half()
     grid = make_rotation_grid(200, 200, 3.7, (2.25, -1.5)).half()
@@ -234,22 +217,17 @@ def test_base_shape_fp16_config4_vs_oracle_and_reference_kernel():
     g2 = grid.permute(0, 2, 3, 1).unsqueeze(1).contiguous().cuda()
     out2 = bt.grid_sampler_chw2(pack_chw(x, 2).cuda(), g2, 256, "bilinear", "zeros", False)
     assert torch.equal(unpack_chw(out2.cpu(), 256), got.cpu())
-    if os.path.exists(REF_LIB):
-        theirs = torch.empty_like(got)
-        dims = lambda t: (ctypes.c_int * 4)(*t.shape)  # noqa: E731
-        _ref_call("ref_grid_sample", 1, ctypes.c_void_p(theirs.data_ptr()), ctypes.c_void_p(xd.data_ptr()),
-                  ctypes.c_void_p(gd.data_ptr()), dims(theirs), dims(xd), dims(gd), 4, 0, 0, 0)
-        e_ref = np.abs(theirs.float().cpu().numpy() - want).max()
-        print(f"\n[grid sampler base fp16] ours {e:.3e}  reference __half kernel {e_ref:.3e} (vs fp32 formulas)")
-        assert e <= e_ref + 1e-6
+    check_digest(REFK, "base_fp16", x, grid)
+    e_ref = float(REFK["base_fp16_err"])
+    print(f"\n[grid sampler base fp16] ours {e:.3e}  reference __half kernel {e_ref:.3e} (vs fp32 formulas)")
+    assert e <= e_ref + 1e-6
 
 
 def test_base_shape_int8_config4_vs_dequant_oracle_and_reference_kernel():
     """BASELINE configs[3], INT8 leg: kCHW4 int8 input [1,256,200,200] and grid with per-tensor scales; ours vs the
     fp32 formulas on the dequantised tensors (at most half an output step: one requantisation), next to the reference's
-    grid_sample_int8 (gridSamplerKernel.cu:2010-2043, :1082-1268: weights quantised to int8 at 1/127, dp4a)."""
-    import ctypes
-
+    grid_sample_int8 (gridSamplerKernel.cu:2010-2043, :1082-1268: weights quantised to int8 at 1/127, dp4a), run on a
+    B200 (REFK)."""
     g = torch.Generator().manual_seed(22)
     x = torch.randn(1, 256, 200, 200, generator=g)
     grid = make_rotation_grid(200, 200, -2.9, (-1.75, 3.0))
@@ -264,17 +242,13 @@ def test_base_shape_int8_config4_vs_dequant_oracle_and_reference_kernel():
     got = unpack_chw(out4.cpu(), 256).float().numpy() * so
     e = np.abs(got - real).max()
     assert e <= 0.5 * so + 1e-6, (e, so)
-    if os.path.exists(REF_LIB):
-        theirs4 = torch.empty_like(out4)
-        d4 = lambda *s: (ctypes.c_int * 4)(*s)  # noqa: E731
-        _ref_call("ref_grid_sample_int8", ctypes.c_void_p(theirs4.data_ptr()), ctypes.c_float(so),
-                  ctypes.c_void_p(x4.data_ptr()), ctypes.c_float(si), ctypes.c_void_p(g4d.data_ptr()),
-                  ctypes.c_float(sg), d4(1, 256, 200, 200), d4(1, 256, 200, 200), d4(1, 2, 200, 200), 4, 0, 0, 0)
-        e_ref = np.abs(unpack_chw(theirs4.cpu(), 256).float().numpy() * so - real).max()
-        print(f"\n[grid sampler base int8] ours {e / so:.3f} LSB  reference grid_sample_int8 {e_ref / so:.3f} LSB")
-        # the reference kernel quantises its bilinear weights to int8 (x127) and requantises twice (:1137-1204): measured
-        # ~30 output steps away from the fp32 formulas at this shape; ours carries the one final rounding
-        assert e <= e_ref + 1e-6
+    check_digest(REFK, "base_int8", iq, gq)
+    assert so == float(REFK["base_int8_so"])
+    e_ref = float(REFK["base_int8_err"])
+    print(f"\n[grid sampler base int8] ours {e / so:.3f} LSB  reference grid_sample_int8 {e_ref / so:.3f} LSB")
+    # the reference kernel quantises its bilinear weights to int8 (x127) and requantises twice (:1137-1204): measured
+    # ~30 output steps away from the fp32 formulas at this shape; ours carries the one final rounding
+    assert e <= e_ref + 1e-6
 
 
 @pytest.mark.parametrize("interp,pad,align", [("bilinear", "zeros", False), ("bilinear", "border", True), ("bicubic", "zeros", False)])

@@ -1,5 +1,5 @@
 """GPU parity tests for RotateTRT / RotateTRT2 (pytest -m gpu). Checkers: oracle/rotate_oracle.c (the reference FP32
-kernel restated), golden vectors from the reference Python binding, and oracle/_ref (the reference's CUDA kernels).
+kernel restated), golden vectors from the reference Python binding and from the reference's CUDA kernels run on a B200.
 Tolerances: source indices bit-exact (given the device's cos/sin); FP32 values 1e-4 against the libm-trig oracle and
 1e-6 against the reference kernel; FP16 1e-3 + output rounding; INT8 half an output step."""
 import ctypes
@@ -14,9 +14,9 @@ import bevformer_tensorrt_b200 as bt
 from bevformer_tensorrt_b200 import _lib
 from bevformer_tensorrt_b200.functions.grid_sampler import pack_chw, unpack_chw
 from bevformer_tensorrt_b200.workloads import quantize_per_tensor
-from oracle import REF_LIB
 from oracle import rotate as orot
-from tests.helpers import GOLDEN, ROTATE_CASES, make_rotate_inputs
+from tests.helpers import (GOLDEN, ROTATE_CASES, check_digest, input_digest, load_ref_kernels, make_rotate_inputs,
+                           sample_index)
 
 pytestmark = pytest.mark.gpu
 
@@ -85,24 +85,29 @@ def test_fp32_matches_reference_golden(case, interp):
     assert d.mean() < 1e-4  # the reference's own acceptance metric and bound (test_rotate.py:98-102, getCost)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_LIB), reason="oracle/_ref not built")
+# the reference's own CUDA kernels, run on a B200 (tests/golden/ref_kernels_rotate.npz, make_golden_ref_kernels.py)
+REFK = load_ref_kernels("rotate")
+
+
 @pytest.mark.parametrize("shape,ang,ctr", [((8, 50, 50), 1.7, (25.0, 25.0)), ((7, 33, 47), 127.3, (20.5, 13.25)),
                                            ((256, 200, 200), -3.3, (100.0, 100.0)),
                                            ((32, 512, 512), 217.9, (500.0, 500.0))])  # fmt: skip
 @pytest.mark.parametrize("interp", ["bilinear", "nearest"])
 def test_fp32_matches_reference_cuda_kernel(shape, ang, ctr, interp):
-    """Same-box A/B with the UNMODIFIED reference kernel: nearest must pick the same pixel everywhere (index
-    arithmetic bit-exact, including the reference's FMA contraction), bilinear agrees to fp32 rounding."""
+    """Against the UNMODIFIED reference kernel: nearest must pick the same pixel everywhere (index arithmetic bit-exact,
+    including the reference's FMA contraction: the whole output's digest), bilinear agrees to fp32 rounding (on a fixed,
+    seeded sample of the output)."""
     g = torch.Generator().manual_seed(11)
-    img = torch.randn(*shape, generator=g).cuda()
-    angle, center = torch.tensor([ang]).cuda(), torch.tensor(list(ctr)).cuda()
-    want = orot.RefRotate().rotate(img, angle, center, IM[interp], "f32")
-    got = bt.rotate(img, angle, center, interp)
-    torch.cuda.synchronize()
+    img = torch.randn(*shape, generator=g)
+    angle, center = torch.tensor([ang]), torch.tensor(list(ctr))
+    key = "fp32_" + "x".join(map(str, shape))
+    check_digest(REFK, key, img, angle, center)
+    got = bt.rotate(img.cuda(), angle.cuda(), center.cuda(), interp).cpu()
     if interp == "nearest":
-        assert torch.equal(got, want)
+        assert input_digest(got) == str(REFK[f"{key}_nearest"])
     else:
-        assert (got - want).abs().max().item() < 1e-6
+        got = got.numpy().reshape(-1)
+        assert np.abs(got[sample_index(got.size, 2048)] - REFK[f"{key}_bilinear"]).max() < 1e-6
 
 
 @pytest.mark.parametrize("case", ["bev_small", "big_angle", "off_center", "odd_c"])
@@ -123,18 +128,17 @@ def test_fp16_and_chw2_match_oracle(case, interp):
     assert torch.equal(unpack_chw(out2[None].cpu(), img.shape[0])[0], got.cpu())
 
 
-@pytest.mark.skipif(not os.path.exists(REF_LIB), reason="oracle/_ref not built")
 def test_fp16_is_closer_to_fp32_truth_than_reference_half_kernel():
     """The reference's __half kernel computes the matrix and coordinates in half precision (rotateKernel.cu:213-260);
-    its own test accepts a mean-abs error of 0.5 (test_rotate.py:104-108). Ours keeps them in fp32."""
+    its own test accepts a mean-abs error of 0.5 (test_rotate.py:104-108). Ours keeps them in fp32. The reference's
+    mean-abs error on these inputs was measured on a B200 (REFK)."""
     g = torch.Generator().manual_seed(3)
     img = torch.randn(16, 200, 200, generator=g)
     angle, center = torch.tensor([3.3]), torch.tensor([100.0, 100.0])
     truth = orot.rotate(img.half().float().numpy(), float(angle.half().float()[0]), center.numpy(), 0)
     ours = bt.rotate(img.half().cuda(), angle.half().cuda(), center.half().cuda(), "bilinear").float().cpu().numpy()
-    theirs = orot.RefRotate().rotate(img.half().cuda(), angle.half().cuda(), center.half().cuda(), 0, "f16")
-    torch.cuda.synchronize()
-    e_ours, e_theirs = np.abs(ours - truth).mean(), np.abs(theirs.float().cpu().numpy() - truth).mean()
+    check_digest(REFK, "fp16", img)
+    e_ours, e_theirs = np.abs(ours - truth).mean(), float(REFK["fp16_mean_err"])
     assert e_ours < 1e-3 and e_ours <= e_theirs, (e_ours, e_theirs)
 
 
@@ -231,11 +235,10 @@ def test_errors_and_edge_cases():
     assert torch.allclose(one, torch.ones(3, 1, 1).cuda())
 
 
-@pytest.mark.skipif(not os.path.exists(REF_LIB), reason="oracle/_ref not built")
 def test_same_box_timing_against_reference_kernel():
-    """Same-box A/B at BEVFormer-base size: device time per call (CUDA events around 20 back-to-back launches) of the
-    reference's rotateKernel<float|__half> and of this library; the numbers go to gpurun_out/rotate_ab.json."""
-    import json
+    """At BEVFormer-base size, device time per call (CUDA events around 20 back-to-back launches) of this library against
+    the reference's rotateKernel<float|__half>, timed the same way on a B200 (REFK: the best of 5 such runs; the card and
+    its power limit are stored with the numbers)."""
 
     def timed(fn, n=20):
         for _ in range(3):
@@ -252,14 +255,11 @@ def test_same_box_timing_against_reference_kernel():
     g = torch.Generator().manual_seed(2)
     img = torch.randn(256, 200, 200, generator=g).cuda()
     angle, center = torch.tensor([2.3]).cuda(), torch.tensor([100.0, 100.0]).cuda()
-    rr = orot.RefRotate()
     res = {}
-    for tag, x, a, c, var in (("f32", img, angle, center, "f32"), ("f16", img.half(), angle.half(), center.half(), "f16")):
-        res[f"reference_{tag}_us"] = timed(lambda: rr.rotate(x, a, c, 0, var))
+    for tag, x, a, c in (("f32", img, angle, center), ("f16", img.half(), angle.half(), center.half())):
+        res[f"reference_{tag}_us"] = float(REFK[f"time_reference_{tag}_us"])
         res[f"b200_{tag}_us"] = timed(lambda: bt.rotate(x, a, c, "bilinear"))
         hwc = x.permute(1, 2, 0).contiguous()
         res[f"b200_hwc_{tag}_us"] = timed(lambda: bt.rotate_hwc(hwc, a, c, "bilinear"))
-    os.makedirs("gpurun_out", exist_ok=True)
-    with open("gpurun_out/rotate_ab.json", "w") as f:
-        json.dump(res, f)
+    print(f"\n[rotate timing] {res} (reference on {REFK['time_device']})")
     assert res["b200_f32_us"] < res["reference_f32_us"] and res["b200_f16_us"] < res["reference_f16_us"], res
