@@ -111,6 +111,11 @@ int b200_grid_sampler_enqueue(const b200_tensor_desc *in, const b200_tensor_desc
   if (nb != 4 && nb != 5) return B200_ERR_BAD_PARAM;
   int id[5], gd[5], od[5];
   for (int i = 0; i < nb; ++i) id[i] = in[0].dims.d[i], gd[i] = in[1].dims.d[i], od[i] = out[0].dims.d[i];
+  // The launcher writes N x C from the input and the spatial extent from the grid, whatever the output descriptor says:
+  // an output that disagrees would be written past its end, so it is rejected before anything is launched.
+  if (in[1].dims.nbDims != nb || out[0].dims.nbDims != nb || od[0] != id[0] || od[1] != id[1]) return B200_ERR_BAD_PARAM;
+  for (int i = 2; i < nb; ++i)
+    if (od[i] != gd[i]) return B200_ERR_BAD_PARAM;
   switch (in[0].type) {
     case 0:
       return b200_grid_sample_f32(static_cast<float *>(outputs[0]), static_cast<const float *>(inputs[0]),
@@ -150,6 +155,14 @@ int b200_grid_sampler_supports_format(int pos, const b200_tensor_desc *io, int n
 // ModulatedDeformableConv2dTRT[2]: enqueue of the reference (…Conv2dPlugin.cpp:117-199). inputs: x, offset, mask,
 // weight[, bias]. stride / padding / dilation are the plugin attributes' int[2]; element [0] goes to the launcher's *_w
 // slot and [1] to *_h exactly as the reference's call does (:152-160). workspace: b200_dcn_enqueue_workspace_size.
+// The launcher derives (Ho, Wo) from those attributes and the kernel size weight.d[2] x weight.d[3]; TensorRT sizes the
+// output from the graph, which may read the attributes the other way round. b200_dcn_enqueue checks the output, offset,
+// mask and weight descriptors against the launcher's geometry and returns B200_ERR_BAD_PARAM if they disagree, instead
+// of letting the kernel read and write past those buffers (the reference does not check).
+static bool dims_are(const b200_tensor_desc &t, int d0, int d1, int d2, int d3) {
+  return t.dims.nbDims == 4 && t.dims.d[0] == d0 && t.dims.d[1] == d1 && t.dims.d[2] == d2 && t.dims.d[3] == d3;
+}
+
 size_t b200_dcn_enqueue_workspace_size(const b200_tensor_desc *in, const int32_t *stride, const int32_t *padding,
                                        const int32_t *dilation, int groups, int deform_groups) {
   if (!in || !stride || !padding || !dilation) return 0;
@@ -172,24 +185,31 @@ int b200_dcn_enqueue(const b200_tensor_desc *in, const b200_tensor_desc *out, co
   const int32_t *x = in[0].dims.d, *w = in[3].dims.d;
   const void *bias = nb_inputs == 5 ? inputs[4] : nullptr;
   const int s0 = stride[0], s1 = stride[1], p0 = padding[0], p1 = padding[1], d0 = dilation[0], d1 = dilation[1];
+  if (in[0].dims.nbDims != 4 || s0 <= 0 || s1 <= 0 || groups <= 0) return B200_ERR_BAD_PARAM;
+  const int kh = w[2], kw = w[3], taps = deform_groups * kh * kw;
+  const int Ho = (x[2] + 2 * p1 - (d1 * (kh - 1) + 1)) / s1 + 1;
+  const int Wo = (x[3] + 2 * p0 - (d0 * (kw - 1) + 1)) / s0 + 1;
+  if (!dims_are(out[0], x[0], w[0], Ho, Wo) || !dims_are(in[1], x[0], 2 * taps, Ho, Wo) ||
+      !dims_are(in[2], x[0], taps, Ho, Wo) || !dims_are(in[3], w[0], x[1] / groups, kh, kw))
+    return B200_ERR_BAD_PARAM;
   switch (in[0].type) {
     case 0:
       return b200_dcn_f32(static_cast<const float *>(inputs[0]), static_cast<const float *>(inputs[3]),
                           static_cast<const float *>(bias), static_cast<const float *>(inputs[1]),
                           static_cast<const float *>(inputs[2]), static_cast<float *>(outputs[0]), workspace, x[0], x[1],
-                          x[2], x[3], w[0], w[3], w[2], s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
+                          x[2], x[3], w[0], kw, kh, s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
     case 1:
       if (in[0].format == 1)
         return b200_dcn_f16_chw2(inputs[0], inputs[3], bias, inputs[1], inputs[2], outputs[0], workspace, x[0], x[1], x[2],
-                                 x[3], w[0], w[3], w[2], s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
+                                 x[3], w[0], kw, kh, s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
       return b200_dcn_f16(inputs[0], inputs[3], bias, inputs[1], inputs[2], outputs[0], workspace, x[0], x[1], x[2], x[3],
-                          w[0], w[3], w[2], s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
+                          w[0], kw, kh, s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
     case 2:
       return b200_dcn_i8(static_cast<const int8_t *>(inputs[0]), in[0].scale, static_cast<const int8_t *>(inputs[3]),
                          in[3].scale, bias, nb_inputs == 5 && in[4].type == 1, static_cast<const int8_t *>(inputs[1]),
                          in[1].scale, static_cast<const int8_t *>(inputs[2]), in[2].scale,
-                         static_cast<int8_t *>(outputs[0]), out[0].scale, workspace, x[0], x[1], x[2], x[3], w[0], w[3],
-                         w[2], s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
+                         static_cast<int8_t *>(outputs[0]), out[0].scale, workspace, x[0], x[1], x[2], x[3], w[0], kw,
+                         kh, s0, s1, p0, p1, d0, d1, groups, deform_groups, x[0], nullptr, stream);
     default:
       return B200_ERR_UNSUPPORTED;
   }

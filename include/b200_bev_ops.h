@@ -471,7 +471,13 @@ int b200_grid_sampler_supports_format(int pos, const b200_tensor_desc *in_out, i
 
 /* ModulatedDeformableConv2dTRT[2] (…Conv2dPlugin.cpp:117-199): inputs = x, offset, mask, weight[, bias] (nb_inputs 4 or
  * 5). stride / padding / dilation = the plugin attributes' int[2]; element [0] is handed to the launcher's *_w slot and
- * [1] to *_h exactly as the reference's enqueue does (:152-160). Dispatch: fp32, fp16 linear, fp16 kCHW2, int8 kCHW4. */
+ * [1] to *_h exactly as the reference's enqueue does (:152-160). Dispatch: fp32, fp16 linear, fp16 kCHW2, int8 kCHW4.
+ * Before launching anything, b200_dcn_enqueue computes (Ho, Wo) as the launcher will (stride / padding / dilation [0]
+ * for w and [1] for h, kernel weight.d[2] x weight.d[3]) and returns B200_ERR_BAD_PARAM unless output == (N, Co, Ho, Wo),
+ * offset == (N, deform_groups*2*kh*kw, Ho, Wo), mask == (N, deform_groups*kh*kw, Ho, Wo) and
+ * weight.d[1] == C / groups: a graph that reads the attributes as (h, w) is refused instead of being read and
+ * written past its buffers. b200_grid_sampler_enqueue likewise requires output == (N, C) of the input followed by the
+ * grid's spatial dims. */
 size_t b200_dcn_enqueue_workspace_size(const b200_tensor_desc *input_desc, const int32_t *stride, const int32_t *padding,
                                        const int32_t *dilation, int groups, int deform_groups);
 int b200_dcn_enqueue(const b200_tensor_desc *input_desc, const b200_tensor_desc *output_desc, const void *const *inputs,
